@@ -55,7 +55,14 @@ def parse():
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the PyTorch-eager CUDA fp32 leg")
     ap.add_argument("--min-warmup", type=int, default=3, help="lower only when profiling under ncu")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU oracle leg (profiling runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned for each file to DIR/<uri>_<output>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 def peaks():
@@ -134,6 +141,19 @@ def workload_config(args, world):
 
 def pool_mode(args, world):
     return world > 1 and args.parallelism in ("auto", "pool")
+
+
+def dump_outputs(outdir, outputs):
+    """Writes the (file, DiarizeOutput) pairs of one step: per file, the speaker turns of both diarizations as
+    (start s, end s, speaker index) rows and the speaker embeddings (one row per speaker, in label order)."""
+    os.makedirs(outdir, exist_ok=True)
+    for file, out in outputs:
+        for name, ann in (("diarization", out.speaker_diarization),
+                          ("exclusive_diarization", out.exclusive_speaker_diarization)):
+            rows = [(s.start, s.end, int(lab.rsplit("_", 1)[1])) for s, _, lab in ann.itertracks(yield_label=True)]
+            np.save(os.path.join(outdir, f"{file['uri']}_{name}.npy"), np.array(rows, dtype=np.float64).reshape(-1, 3))
+        np.save(os.path.join(outdir, f"{file['uri']}_speaker_embeddings.npy"),
+                np.asarray(out.speaker_embeddings, dtype=np.float64))
 
 
 def cpu_pass(seconds, models, seed=4242):
@@ -301,12 +321,11 @@ def main():
     resident = pool.upload(files) if use_pool else pipe.upload(files)
     done = [0]
     coll_ms = []
+    last_outputs = []
 
     def step_resident():
-        n = 0
-        for _ in (pool.run_resident(resident) if use_pool else pipe.run_resident(resident)):
-            n += 1
-        done[0] = n
+        last_outputs[:] = pool.run_resident(resident) if use_pool else pipe.run_resident(resident)
+        done[0] = len(last_outputs)
         if use_pool:
             coll_ms.append(pool._events)
 
@@ -353,6 +372,8 @@ def main():
     if world > 1:
         dist.all_reduce(files_done)
     assert int(files_done.item()) == world * nfiles, "every file must come out of the per-file stage exactly once"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_outputs)
     ms_e2e = timed(step_e2e, max(1, args.steps))
     value = world * audio_hours / (ms_resident / 1e3)
     e2e = world * audio_hours / (ms_e2e / 1e3)

@@ -50,15 +50,19 @@ gamma, pi = ref["vbx"].cluster_vbx(ahc, fea, phi, Fa=0.07, Fb=0.8, maxIters=20)
 out["vbx_fea"], out["vbx_phi"], out["vbx_ahc"], out["vbx_gamma"], out["vbx_pi"] = fea, phi, ahc, gamma, pi
 plda = syn.make_plda(2)
 import tempfile, os
-with tempfile.TemporaryDirectory() as td:
+from threadpoolctl import threadpool_limits
+
+# the PLDA setup (inverses, generalised eigh) rounds differently with the number of BLAS threads: one thread here and
+# in tests/test_oracle_golden.py, so that the comparison does not depend on the host's core count
+with tempfile.TemporaryDirectory() as td, threadpool_limits(limits=1):
     np.savez(os.path.join(td, "xvec_transform.npz"), mean1=plda["mean1"], mean2=plda["mean2"], lda=plda["lda"])
     np.savez(os.path.join(td, "plda.npz"), mu=plda["mu"], tr=plda["tr"], psi=plda["psi"])
     xvec_tf, plda_tf, plda_psi = ref["vbx"].vbx_setup(os.path.join(td, "xvec_transform.npz"),
                                                       os.path.join(td, "plda.npz"))
-emb = rng.standard_normal((7, 256))
-out["plda_in"] = emb
-out["plda_out"] = plda_tf(xvec_tf(emb), lda_dim=128)
-out["plda_psi"] = plda_psi
+    emb = rng.standard_normal((7, 256))
+    out["plda_in"] = emb
+    out["plda_out"] = plda_tf(xvec_tf(emb), lda_dim=128)
+    out["plda_psi"] = plda_psi
 
 # ---- ResNet34 trunk + TSTP + seg_1 (models/embedding/wespeaker/resnet.py) --------------------------------------
 net = ref["resnet"].ResNet34(80, 256, pooling_func="TSTP", two_emb_layer=False)

@@ -75,7 +75,11 @@ def test_audio_matches_reference_io(ref):
     from pyannote_audio_b200.audio import Audio
     from pyannote_audio_b200.core import Segment
 
-    stereo, hi = torch.from_numpy(ref["io_stereo"]), torch.from_numpy(ref["io_hi"])
+    g = torch.Generator().manual_seed(5)                 # the generator's stereo input, drawn from the same seed
+    stereo = torch.rand(2, 24000, generator=g) * 2 - 1
+    assert np.array_equal(stereo[:, :64].numpy(), ref["io_stereo_head"])
+    assert stereo.double().sum().item() == float(ref["io_stereo_sum"])
+    hi = torch.from_numpy(ref["io_hi"])
     a16 = Audio(sample_rate=16000, mono="downmix")
     w, sr = a16({"waveform": stereo, "sample_rate": 16000})
     assert sr == 16000 and np.array_equal(w.numpy(), ref["io_downmix"])
